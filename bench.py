@@ -15,6 +15,8 @@ One JSON line on stdout (rank 0):
   roofline       dominant kernel: algorithmic bytes / CUDA-event duration against the measured HBM peak
   cpu_baseline   the CPU port of the reference algorithm on a bounded sample (rank 0, N = 1)
   --impl reference   times that CPU port alone (rank 0 only), same JSON contract
+  --dump-outputs DIR   after the timed steps, rank 0 writes what the device-resident timed path computed in its last
+                       step (images, radii, parameter gradients / fused features) to DIR/<name>.npy; see dump_outputs()
 """
 from __future__ import annotations
 
@@ -394,6 +396,34 @@ def fma_roofline(C, blended_pairs, per_stage):
 
 
 # ------------------------------------------------------------------------------ GPU arm: shared pieces
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(path, arrays):
+    """Write each output tensor as path/<name>.npy: float32 when it is floating point, float64 otherwise (exact for
+    the integer and boolean outputs).  Together the files stay within DUMP_BYTES: an output with more elements than
+    its share is written as the flat values at a fixed seeded sample of positions (the same positions for every
+    output of that size), so two builds run with the same arguments can be compared output for output."""
+    import torch
+    os.makedirs(path, exist_ok=True)
+    cap = DUMP_BYTES // 8 // max(len(arrays), 1)
+    for name, t in arrays.items():
+        t = t.detach()
+        if t.numel() > cap:
+            idx = np.unique(np.random.default_rng(t.numel()).integers(0, t.numel(), cap))
+            t = t.reshape(-1)[torch.as_tensor(idx, device=t.device)]
+        t = t.to(torch.float32 if t.is_floating_point() else torch.float64)
+        np.save(os.path.join(path, f"{name}.npy"), t.cpu().numpy())
+
+
+def render_outputs(out, prefix=""):
+    """The tensors a render()/render_chn() call hands its caller (viewspace_points through its gradient)."""
+    d = {prefix + k: v for k, v in out.items() if k != "viewspace_points"}
+    if out["viewspace_points"].grad is not None:
+        d[prefix + "viewspace_points_grad"] = out["viewspace_points"].grad
+    return d
+
+
 class Pipe:
     convert_shs_python = False
     compute_cov3d_python = False
@@ -594,13 +624,19 @@ def run_k3(args, rank, world, local_rank):
         # and at every step the `world` ranks render `world` DIFFERENT views
         return (i + rank) % NVIEWS
 
-    def step_device(i, exchange=True):
+    last = {}
+
+    def step_device(i, exchange=True, keep=False):
         out = render_chn(cams[view_of(i)], pc, Pipe, bg, num_channels=C, override_color=feats)
         if overlap is not None:
             overlap.arm(feats)
         out["render"].backward(dL_fixed)
         if exchange:
             allreduce_grads()
+        if keep:
+            last.update(render_outputs(out))
+            last.update({f"{n}_grad": p.grad for n, p in zip(("features", "xyz", "scaling", "rotation", "opacity"),
+                                                              params)})
         zero_grads()
 
     cam_dev = Cam()
@@ -701,7 +737,11 @@ def run_k3(args, rank, world, local_rank):
     stats = view_stats(h, cfg, pc, feats, cams[rank % NVIEWS], bg)
 
     # ---- device-resident timed region (stage tracing + clock sampling), then the same without the exchange
-    ms_dev, ms_mine, per_stage, _, clocks, launches = h.profiled(step_device, args.steps)
+    ms_dev, ms_mine, per_stage, _, clocks, launches = h.profiled(
+        lambda i: step_device(i, keep=args.dump_outputs is not None and i == args.steps - 1), args.steps)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, last)
+    last.clear()
     rank_ms = h.gather_floats(ms_mine / args.steps)
     ms_nocomm = None
     if world > 1:
@@ -858,9 +898,13 @@ def run_k2(args, rank, world, local_rank):
     bg = torch.zeros(3, device=dev)
     cams = [h.dev_cam(c) for c in cams_np]
 
-    def step_device(i):
+    last = {}
+
+    def step_device(i, keep=False):
         with torch.no_grad():
-            render(cams[(i + rank) % NVIEWS], pc, Pipe, bg)
+            out = render(cams[(i + rank) % NVIEWS], pc, Pipe, bg)
+        if keep:
+            last.update(render_outputs(out))
 
     host_cam = [torch.from_numpy(np.concatenate([c.world_view_transform.ravel(), c.full_proj_transform.ravel(),
                                                  c.camera_center.ravel()]).astype(np.float32)).pin_memory()
@@ -887,7 +931,11 @@ def run_k2(args, rank, world, local_rank):
     for i in range(h.warmup):
         step_device(i)
     stats = view_stats(h, cfg, pc, None, cams[rank % NVIEWS], bg)
-    ms_dev, ms_mine, per_stage, _, clocks, launches = h.profiled(step_device, args.steps)
+    ms_dev, ms_mine, per_stage, _, clocks, launches = h.profiled(
+        lambda i: step_device(i, keep=args.dump_outputs is not None and i == args.steps - 1), args.steps)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, last)
+    last.clear()
     for i in range(2):
         step_e2e(i)
     ms_e2e, _ = h.timed(step_e2e, args.steps, finish=lambda i: img_ev[i % 2].synchronize())
@@ -969,16 +1017,24 @@ def run_k4(args, rank, world, local_rank):
         dist.all_reduce(small)
         overlap.finish()
 
-    def step_device(i, batched=True, do_exchange=True):
+    last = {}
+
+    def step_device(i, batched=True, do_exchange=True, keep=False):
         for sub in subs:
             if batched:
                 outs = render_chn_batch([cams[k] for k in sub], pc, Pipe, bg, num_channels=C, override_color=feats)
                 torch.autograd.backward([o["render"] for o in outs], [dL_fixed] * len(outs))
+                if keep:
+                    for k, o in zip(sub, outs):
+                        last.update(render_outputs(o, f"view{k:02d}_"))
             else:
                 for k in sub:
                     render_chn(cams[k], pc, Pipe, bg, num_channels=C, override_color=feats)["render"].backward(dL_fixed)
         if do_exchange:
             exchange()
+        if keep:
+            last.update({f"{n}_grad": p.grad for n, p in zip(("features", "xyz", "scaling", "rotation", "opacity"),
+                                                              params)})
         zero_grads()
 
     rng = np.random.default_rng(99 + rank)
@@ -1022,7 +1078,11 @@ def run_k4(args, rank, world, local_rank):
     torch.cuda.synchronize(dev)
     stats = view_stats(h, cfg, pc, feats, cams[mine[0]], bg)
     steps = args.steps
-    ms_dev, ms_mine, per_stage, counts, clocks, launches = h.profiled(step_device, steps)
+    ms_dev, ms_mine, per_stage, counts, clocks, launches = h.profiled(
+        lambda i: step_device(i, keep=args.dump_outputs is not None and i == steps - 1), steps)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, last)
+    last.clear()
     rank_ms = h.gather_floats(ms_mine / steps)
     ms_nc, _ = h.timed(lambda i: step_device(i, do_exchange=False), steps)
     nloop = max(1, steps // 2)
@@ -1149,6 +1209,8 @@ def run_k5(args, rank, world, local_rank):
     nvis = [int(v) for v in nvis_acc]
     steps = args.steps
     ms_dev, ms_mine, per_stage, counts, clocks, launches = h.profiled(step_device, steps)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"fused_features": fs, "counts": cnt})   # the last step's, untouched since
     rank_ms = h.gather_floats(ms_mine / steps)
 
     def no_exchange(i):
@@ -1221,7 +1283,14 @@ def main():
     ap.add_argument("--config", default="K3", choices=sorted(CONFIGS))
     ap.add_argument("--no-baselines", action="store_true", help="skip the reference-CUDA and CPU legs")
     ap.add_argument("--quick", action="store_true", help="skip the per-view cost spread")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the timed path computed in its last step to DIR/<name>.npy (float32 / float64, "
+                         "64 MB at most: larger outputs as a fixed seeded sample of their values)")
     args = ap.parse_args()
+    if args.steps is not None and args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs is not None and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of the CUDA path (--impl ours)")
     claim_stdout()
     if args.steps is None:
         args.steps = {"K2": 40, "K3": 20, "K4": 3, "K5": 3}[args.config] if args.impl == "ours" else 2

@@ -1,9 +1,9 @@
 """Generates tests/golden/fusion_golden.npz by running the REFERENCE's own
-PointCloudToImageMapper.compute_mapping (imported from /root/reference/dataset/fusion_utils.py, with
-the collections.Sequence/Iterable aliases it needs on Python >= 3.10) and the accumulate/normalise
-statements of fusion.py:136-147 on seeded synthetic inputs.  Run in the build container:
+PointCloudToImageMapper.compute_mapping (imported from dataset/fusion_utils.py of the original project's
+source tree, with the collections.Sequence/Iterable aliases it needs on Python >= 3.10) and the
+accumulate/normalise statements of fusion.py:136-147 on seeded synthetic inputs:
 
-    python tests/golden/make_fusion_golden.py
+    SGB_REFERENCE_TREE=<original project> python tests/golden/make_fusion_golden.py
 
 Inputs are regenerated from the seed by the tests; only outputs are stored."""
 import collections
@@ -16,7 +16,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 sys.path.insert(0, ROOT)
-REF = "/root/reference"
+REF = os.environ.get("SGB_REFERENCE_TREE", "")
 
 
 def import_reference_mapper():

@@ -41,3 +41,33 @@ def test_stray_writes_to_fd1_do_not_reach_stdout(tmp_path):
     assert p.returncode == 0, p.stderr[-1000:]
     assert p.stdout == '{"ok": 1}\n'
     assert "NCCL version" in p.stderr and "python print too" in p.stderr
+
+
+@pytest.mark.parametrize("argv", [["--steps", "0"], ["--impl", "reference", "--dump-outputs", "out"]])
+def test_unusable_arguments_are_refused(argv):
+    p = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), *argv], capture_output=True, text=True,
+                       timeout=120, cwd=ROOT)
+    assert p.returncode == 2 and p.stdout == "", p.stderr[-1000:]
+
+
+def test_dump_outputs_writes_each_output_within_the_budget(tmp_path):
+    """--dump-outputs: one <name>.npy per output, float32 for floating point and float64 for the rest; whole while an
+    output fits its share of the 64 MB, beyond that the values at sample positions fixed by the output's size."""
+    import numpy as np
+    import torch
+    sys.path.insert(0, ROOT)
+    import bench
+    outs = {"render": torch.arange(10_000_000, dtype=torch.float32).reshape(10, 1000, 1000),
+            "radii": torch.arange(7, dtype=torch.int32), "visibility_filter": torch.tensor([True, False])}
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), outs)
+    files = sorted(os.listdir(tmp_path / "a"))
+    assert files == ["radii.npy", "render.npy", "visibility_filter.npy"]
+    assert sum(os.path.getsize(tmp_path / "a" / f) for f in files) <= bench.DUMP_BYTES
+    render = np.load(tmp_path / "a" / "render.npy")
+    assert render.dtype == np.float32 and render.ndim == 1 and 0 < render.size < 10_000_000
+    assert np.all(np.diff(render) > 0)                       # distinct positions in order: the values are the indices
+    assert np.array_equal(render, np.load(tmp_path / "b" / "render.npy"))
+    radii = np.load(tmp_path / "a" / "radii.npy")
+    assert radii.dtype == np.float64 and np.array_equal(radii, np.arange(7))
+    assert np.array_equal(np.load(tmp_path / "a" / "visibility_filter.npy"), [1.0, 0.0])

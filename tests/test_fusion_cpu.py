@@ -11,6 +11,7 @@ sys.path.insert(0, os.path.join(os.path.dirname(os.path.abspath(__file__)), "gol
 from make_fusion_golden import fusion_inputs  # noqa: E402
 
 from oracle import fusion_oracle as fo  # noqa: E402
+from reference_data import Reference  # noqa: E402
 
 GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "fusion_golden.npz")
 
@@ -47,15 +48,20 @@ def test_some_points_visible_and_some_not(data):
         assert 0 < vis.sum() < vis.size
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference"), reason="reference tree not mounted")
 def test_oracle_matches_live_reference_on_other_seed():
-    from make_fusion_golden import import_reference_mapper
-    Mapper = import_reference_mapper()
+    """Other seed, sizes and thresholds than fusion_golden.npz; the reference mapper's output is stored in
+    tests/golden/reference_outputs.npz (recorded with SGB_RECORD_REFERENCE, see tests/reference_data.py)."""
+    ref = Reference("fusion_mapping_seed7")
+    if ref.recording:
+        from make_fusion_golden import import_reference_mapper
+        Mapper = import_reference_mapper()
     scene, cams, feats, depths = fusion_inputs(seed=7, P=5000, w=96, h=64, C=4, nviews=2)
     for i, cam in enumerate(cams):
-        for depth in (None, "surface", depths[i]):
-            ref = Mapper([96, 64], 0.1, 2, cam.intrinsics())
-            want, _ = ref.compute_mapping(cam.world_view_transform, scene.xyz, depth)
+        for mode, depth in zip(("none", "surface", "depth"), (None, "surface", depths[i])):
+            if ref.recording:
+                want, _ = Mapper([96, 64], 0.1, 2, cam.intrinsics()).compute_mapping(cam.world_view_transform,
+                                                                                     scene.xyz, depth)
+                ref.put(f"{mode}_mapping_{i}", want)
             K = fo.rescale_intrinsics(cam.intrinsics(), [96, 64])
             got = fo.compute_mapping(cam.world_view_transform, scene.xyz, [96, 64], K, 0.1, 2, depth)
-            assert np.array_equal(got, want)
+            assert ref.equal(f"{mode}_mapping_{i}", got), (mode, i)

@@ -1,5 +1,6 @@
-"""distCUDA2 (SURVEY §8 n4): csrc/knn.cu against the compiled unmodified reference simple-knn (bit-exact) and
-against the numpy brute-force oracle."""
+"""distCUDA2 (SURVEY §8 n4): csrc/knn.cu against the compiled unmodified reference simple-knn (bit-exact; its outputs
+are stored in tests/golden/reference_outputs.npz, see tests/reference_data.py) and against the numpy brute-force
+oracle."""
 import ctypes as C
 import os
 import sys
@@ -10,6 +11,9 @@ import torch
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
+sys.path.insert(0, os.path.join(ROOT, "tests"))
+from reference_data import Reference  # noqa: E402
+
 pytestmark = pytest.mark.gpu
 REF = os.path.join(ROOT, "oracle", "_ref", "libref_knn.so")
 
@@ -27,6 +31,7 @@ def _clouds(n, seed):
 
 
 def _ref(points_dev):
+    """The live reference library: only recording runs (SGB_RECORD_REFERENCE) call it."""
     lib = C.CDLL(REF)
     lib.ref_knn.argtypes = [C.c_int, C.c_void_p, C.c_void_p]
     out = torch.zeros(points_dev.shape[0], device=points_dev.device)
@@ -34,15 +39,17 @@ def _ref(points_dev):
     return out
 
 
-@pytest.mark.skipif(not os.path.exists(REF), reason="oracle/_ref/libref_knn.so not built")
 @pytest.mark.parametrize("n", [5, 300, 20000, 200001])
 def test_bit_exact_vs_compiled_reference(n):
     from semantic_gaussians_b200.simple_knn._C import distCUDA2
     dev = torch.device("cuda:0")
+    ref = Reference(f"knn[{n}]")
     for name, pts in _clouds(n, n).items():
         p = torch.from_numpy(pts).to(dev)
-        ours, ref = distCUDA2(p), _ref(p)
-        assert torch.equal(ours, ref), (name, n, float((ours - ref).abs().max()))
+        if ref.recording:
+            ref.put(name, _ref(p))
+        ours = distCUDA2(p)
+        assert ref.equal(name, ours), (name, n)
 
 
 @pytest.mark.parametrize("n", [4, 7, 257, 1500])

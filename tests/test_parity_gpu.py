@@ -1,6 +1,7 @@
 """Parity of the CUDA path (through the drop-in Python API over the C-ABI) against
-  (a) the UNMODIFIED compiled reference run live on the same GPU (oracle/_ref) — bit-exact for the
-      integer stage and, on the RGB-D path, for the pixels too; 1e-4 relative for floats;
+  (a) the UNMODIFIED compiled reference (oracle/_ref) on the same inputs, its outputs stored in
+      tests/golden/reference_outputs.npz (tests/reference_data.py) — bit-exact for the integer stage and, on the
+      RGB-D path, for the pixels too; 1e-4 relative for floats;
   (b) golden fixtures produced by that reference (tests/golden/raster_golden_k1.npz);
   (c) the CPU oracle (oracle/raster_oracle.c)."""
 import os
@@ -11,7 +12,8 @@ import pytest
 import torch
 
 sys.path.insert(0, os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden"))
-from util import dev_cam, dev_scene, frac_bad, ours_state, rel_err, run_ours  # noqa: E402
+from reference_data import Reference  # noqa: E402
+from util import dev_cam, dev_scene, frac_bad, ours_state, run_ours  # noqa: E402
 
 from semantic_gaussians_b200.scene_synth import make_scene, orbit_cameras  # noqa: E402
 
@@ -21,9 +23,8 @@ RTOL = 1e-4   # north_star: "within 1e-4 rel fp32"
 
 
 def _ref(name):
+    """The live reference library: only recording runs (SGB_RECORD_REFERENCE) call it."""
     from oracle import ref as refmod
-    if not refmod.available(name):
-        pytest.skip(f"oracle/_ref/libref_{name}.so not built")
     return refmod.RefRasterizer(name)
 
 
@@ -33,10 +34,6 @@ def _ref_forward(r, sc, cm, C, use_features, bg):
                      W=cm["W"], H=cm["H"], shs=None if use_features else sc["shs"],
                      colors_precomp=sc["features"] if use_features else None, scales=sc["scales"],
                      rotations=sc["rotations"], num_channels=C)
-
-
-def _bits(t):
-    return t.contiguous().view(torch.int32)
 
 
 @pytest.mark.parametrize("P,W,H,view", [(10000, 256, 256, 0), (200000, 640, 480, 2), (1000000, 1920, 1080, 1),
@@ -49,20 +46,29 @@ def test_rgbd_forward_bit_exact_vs_reference(P, W, H, view):
     cam = orbit_cameras(4, W, H)[view]
     sc, cm = dev_scene(scene, dev), dev_cam(cam, dev)
     st = ours_state(sc, cm, 3, use_features=False, want_depth=True)
-    r = _ref("rgbd")
-    out = _ref_forward(r, sc, cm, 3, False, torch.zeros(3, device=dev))
-    vis = out["radii"] > 0
-    assert st["R"] == out["R"]
-    assert torch.equal(st["radii"], out["radii"])
-    for name in ("depths", "means2D", "conic_opacity", "cov3D", "rgb", "tiles_touched"):
-        assert torch.equal(_bits(st[name][vis]), _bits(r.field(name)[vis])), name
-    assert torch.equal(st["clamped"][vis], r.field("clamped")[vis])
-    assert torch.equal(st["point_list"], r.field("point_list"))          # sort order incl. tie-breaks
-    assert torch.equal(st["ranges"], r.field("ranges"))
-    assert torch.equal(st["n_contrib"], r.field("n_contrib"))
-    assert torch.equal(_bits(st["final_T"]), _bits(r.field("accum_alpha")))
-    assert torch.equal(_bits(st["color"]), _bits(out["color"]))
-    assert torch.equal(_bits(st["depth"]), _bits(out["depth"]))
+    ref = Reference(f"rgbd_forward[{P}-{W}-{H}-{view}]")
+    if ref.recording:
+        r = _ref("rgbd")
+        out = _ref_forward(r, sc, cm, 3, False, torch.zeros(3, device=dev))
+        rvis = out["radii"] > 0
+        for name in ("R", "radii", "color", "depth"):
+            ref.put(name, out[name])
+        for name in ("depths", "means2D", "conic_opacity", "cov3D", "rgb", "tiles_touched", "clamped"):
+            ref.put(name, r.field(name)[rvis])
+        for name in ("point_list", "ranges", "n_contrib", "accum_alpha"):
+            ref.put(name, r.field(name))
+        del out, r
+    assert ref.equal("R", st["R"])
+    assert ref.equal("radii", st["radii"])
+    vis = st["radii"] > 0                                              # == the reference's mask (radii equal)
+    for name in ("depths", "means2D", "conic_opacity", "cov3D", "rgb", "tiles_touched", "clamped"):
+        assert ref.equal(name, st[name][vis]), name                     # bits of the floats
+    assert ref.equal("point_list", st["point_list"])                  # sort order incl. tie-breaks
+    assert ref.equal("ranges", st["ranges"])
+    assert ref.equal("n_contrib", st["n_contrib"])
+    assert ref.equal("accum_alpha", st["final_T"])
+    assert ref.equal("color", st["color"])
+    assert ref.equal("depth", st["depth"])
 
 
 @pytest.mark.parametrize("P,W,H,C", [(100000, 640, 480, 32), (100000, 640, 480, 100), (50000, 320, 240, 5),
@@ -74,16 +80,23 @@ def test_channel_forward_vs_reference(P, W, H, C):
     cam = orbit_cameras(4, W, H)[1]
     sc, cm = dev_scene(scene, dev), dev_cam(cam, dev)
     st = ours_state(sc, cm, C, use_features=True)
-    r = _ref("chn")
-    out = _ref_forward(r, sc, cm, C, True, torch.zeros(C, device=dev))
-    assert st["R"] == out["R"]
-    assert torch.equal(st["radii"], out["radii"])
-    assert torch.equal(st["point_list"], r.field("point_list"))
-    assert torch.equal(st["ranges"], r.field("ranges"))
-    assert torch.equal(st["n_contrib"], r.field("n_contrib"))
-    assert torch.equal(_bits(st["final_T"]), _bits(r.field("accum_alpha")))
-    assert frac_bad(st["color"], out["color"], rtol=RTOL, atol_scale=1e-6) == 0.0
-    assert rel_err(st["color"], out["color"]) < 1e-5
+    ref = Reference(f"channel_forward[{P}-{W}-{H}-{C}]")
+    if ref.recording:
+        r = _ref("chn")
+        out = _ref_forward(r, sc, cm, C, True, torch.zeros(C, device=dev))
+        for name in ("R", "radii", "color"):
+            ref.put(name, out[name])
+        for name in ("point_list", "ranges", "n_contrib", "accum_alpha"):
+            ref.put(name, r.field(name))
+        del out, r
+    assert ref.equal("R", st["R"])
+    assert ref.equal("radii", st["radii"])
+    assert ref.equal("point_list", st["point_list"])
+    assert ref.equal("ranges", st["ranges"])
+    assert ref.equal("n_contrib", st["n_contrib"])
+    assert ref.equal("accum_alpha", st["final_T"])
+    assert ref.frac_bad("color", st["color"], rtol=RTOL, atol_scale=1e-6) == 0.0
+    assert ref.rel_err("color", st["color"]) < 1e-5
 
 
 @pytest.mark.parametrize("refname,P,W,H,C,use_features", [
@@ -102,19 +115,24 @@ def test_backward_vs_reference(refname, P, W, H, C, use_features):
     o = run_ours("rgbd" if refname == "rgbd" else "chn", sc, cm, bg, use_features=use_features)
     dL = torch.as_tensor(np.random.default_rng(5).standard_normal((C, H, W)).astype(np.float32), device=dev)
     (o["color"] * dL).sum().backward()
-    r = _ref(refname)
-    sd = {k: (v.detach() if v is not None else None) for k, v in sc.items()}
-    _ref_forward(r, sd, cm, C, use_features, bg)
-    g = r.backward(dL)
     pairs = [("dL_dmeans2D", o["means2D"].grad), ("dL_dopacity", sc["opacities"].grad.view(-1)),
              ("dL_dmeans3D", sc["means3D"].grad), ("dL_dscales", sc["scales"].grad),
              ("dL_drotations", sc["rotations"].grad)]
     pairs.append(("dL_dcolors", sc["features"].grad) if use_features else ("dL_dsh", sc["shs"].grad))
+    ref = Reference(f"backward[{refname}-{P}-{W}-{H}-{C}-{use_features}]")
+    if ref.recording:
+        r = _ref(refname)
+        sd = {k: (v.detach() if v is not None else None) for k, v in sc.items()}
+        _ref_forward(r, sd, cm, C, use_features, bg)
+        g = r.backward(dL)
+        for name, _ in pairs:
+            ref.put(name, g[name])
+        del r, g
     for name, got in pairs:
         # the reference itself sums with fp32 atomics in arbitrary order: compare at 1e-4 relative
-        # plus 1e-4 of the tensor's scale, and require every entry to pass
-        assert frac_bad(got, g[name], rtol=RTOL, atol_scale=1e-4) == 0.0, name
-        assert rel_err(got, g[name]) < 1e-4, name
+        # plus 1e-4 of the tensor's scale, and require every stored entry to pass
+        assert ref.frac_bad(name, got, rtol=RTOL, atol_scale=1e-4) == 0.0, name
+        assert ref.rel_err(name, got) < 1e-4, name
 
 
 def test_cov3d_precomp_and_scale_modifier_vs_reference():
@@ -126,19 +144,26 @@ def test_cov3d_precomp_and_scale_modifier_vs_reference():
     pc = GaussianModel.from_activated(scene.xyz, scene.scales, scene.rotations, scene.opacity, scene.shs, device=dev)
     cov = pc.get_covariance(1.7).contiguous()
     o = run_ours("rgbd", sc, cm, torch.zeros(3, device=dev), use_features=False, cov3D_precomp=cov)
-    r = _ref("rgbd")
-    out = r.forward(bg=torch.zeros(3, device=dev), means3D=sc["means3D"], opacities=sc["opacities"],
-                    viewmatrix=cm["viewmatrix"], projmatrix=cm["projmatrix"], campos=cm["campos"],
-                    tanfovx=cm["tanfovx"], tanfovy=cm["tanfovy"], W=320, H=240, shs=sc["shs"], cov3D_precomp=cov)
-    assert torch.equal(o["radii"], out["radii"])
-    assert torch.equal(_bits(o["color"]), _bits(out["color"]))
     o2 = run_ours("rgbd", sc, cm, torch.zeros(3, device=dev), use_features=False, scale_modifier=0.6)
-    out2 = r.forward(bg=torch.zeros(3, device=dev), means3D=sc["means3D"], opacities=sc["opacities"],
-                     viewmatrix=cm["viewmatrix"], projmatrix=cm["projmatrix"], campos=cm["campos"],
-                     tanfovx=cm["tanfovx"], tanfovy=cm["tanfovy"], W=320, H=240, shs=sc["shs"], scales=sc["scales"],
-                     rotations=sc["rotations"], scale_modifier=0.6)
-    assert torch.equal(_bits(o2["color"]), _bits(out2["color"]))
-    assert torch.equal(_bits(o2["depth"]), _bits(out2["depth"]))
+    ref = Reference("cov3d_precomp_and_scale_modifier")
+    if ref.recording:
+        r = _ref("rgbd")
+        out = r.forward(bg=torch.zeros(3, device=dev), means3D=sc["means3D"], opacities=sc["opacities"],
+                        viewmatrix=cm["viewmatrix"], projmatrix=cm["projmatrix"], campos=cm["campos"],
+                        tanfovx=cm["tanfovx"], tanfovy=cm["tanfovy"], W=320, H=240, shs=sc["shs"], cov3D_precomp=cov)
+        ref.put("cov3D_precomp.radii", out["radii"])
+        ref.put("cov3D_precomp.color", out["color"])
+        out2 = r.forward(bg=torch.zeros(3, device=dev), means3D=sc["means3D"], opacities=sc["opacities"],
+                         viewmatrix=cm["viewmatrix"], projmatrix=cm["projmatrix"], campos=cm["campos"],
+                         tanfovx=cm["tanfovx"], tanfovy=cm["tanfovy"], W=320, H=240, shs=sc["shs"], scales=sc["scales"],
+                         rotations=sc["rotations"], scale_modifier=0.6)
+        ref.put("scale_modifier.color", out2["color"])
+        ref.put("scale_modifier.depth", out2["depth"])
+        del out, out2, r
+    assert ref.equal("cov3D_precomp.radii", o["radii"])
+    assert ref.equal("cov3D_precomp.color", o["color"])
+    assert ref.equal("scale_modifier.color", o2["color"])
+    assert ref.equal("scale_modifier.depth", o2["depth"])
 
 
 def test_mark_visible_vs_reference_and_oracle():
@@ -263,17 +288,21 @@ def test_empty_and_degenerate_inputs():
 def test_sh_degrees_and_ragged_image_sizes():
     dev = torch.device("cuda:0")
     scene = make_scene(20000, seed=21, sh=True)
-    r = _ref("rgbd")
+    ref = Reference("sh_degrees_and_ragged_image_sizes")
     for deg, (W, H) in zip((0, 1, 2, 3), ((17, 33), (250, 100), (641, 479), (16, 16))):
         cam = orbit_cameras(2, W, H)[1]
         sc, cm = dev_scene(scene, dev), dev_cam(cam, dev)
         o = run_ours("rgbd", sc, cm, torch.zeros(3, device=dev), use_features=False, sh_degree=deg)
-        out = r.forward(bg=torch.zeros(3, device=dev), means3D=sc["means3D"], opacities=sc["opacities"],
-                        viewmatrix=cm["viewmatrix"], projmatrix=cm["projmatrix"], campos=cm["campos"],
-                        tanfovx=cm["tanfovx"], tanfovy=cm["tanfovy"], W=W, H=H, shs=sc["shs"], scales=sc["scales"],
-                        rotations=sc["rotations"], sh_degree=deg)
-        assert torch.equal(_bits(o["color"]), _bits(out["color"])), (deg, W, H)
-        assert torch.equal(_bits(o["depth"]), _bits(out["depth"]))
+        if ref.recording:
+            out = _ref("rgbd").forward(
+                bg=torch.zeros(3, device=dev), means3D=sc["means3D"], opacities=sc["opacities"],
+                viewmatrix=cm["viewmatrix"], projmatrix=cm["projmatrix"], campos=cm["campos"], tanfovx=cm["tanfovx"],
+                tanfovy=cm["tanfovy"], W=W, H=H, shs=sc["shs"], scales=sc["scales"], rotations=sc["rotations"],
+                sh_degree=deg)
+            ref.put(f"color.{deg}", out["color"])
+            ref.put(f"depth.{deg}", out["depth"])
+        assert ref.equal(f"color.{deg}", o["color"]), (deg, W, H)
+        assert ref.equal(f"depth.{deg}", o["depth"])
 
 
 def test_channel_forward_and_backward_above_65535_tiles():
@@ -285,11 +314,15 @@ def test_channel_forward_and_backward_above_65535_tiles():
     sc, cm = dev_scene(scene, dev, requires_grad=True), dev_cam(cam, dev)
     bg = torch.linspace(0.0, 0.3, C, device=dev)
     o = run_ours("chn", sc, cm, bg, use_features=True)
-    r = _ref("chn")
     sd = {k: (v.detach() if v is not None else None) for k, v in sc.items()}
-    out = _ref_forward(r, sd, cm, C, True, bg)
-    assert torch.equal(o["radii"], out["radii"])
-    assert rel_err(o["color"], out["color"]) < 1e-5
+    ref = Reference("channel_forward_above_65535_tiles")
+    if ref.recording:
+        out = _ref_forward(_ref("chn"), sd, cm, C, True, bg)
+        ref.put("radii", out["radii"])
+        ref.put("color", out["color"])
+        del out
+    assert ref.equal("radii", o["radii"])
+    assert ref.rel_err("color", o["color"]) < 1e-5
     dL = torch.zeros((C, H, W), device=dev)
     dL[:, ::7, ::5] = 1.0
     (o["color"] * dL).sum().backward()
@@ -315,9 +348,14 @@ def test_channel_counts_not_multiple_of_four_and_ragged_images(C, W, H):
     bg = torch.linspace(0.1, 0.4, C, device=dev)
     o = run_ours("chn", sc, cm, bg, use_features=True)
     sd = {k: (v.detach() if v is not None else None) for k, v in sc.items()}
-    out = _ref_forward(_ref("chn"), sd, cm, C, True, bg)
-    assert torch.equal(o["radii"], out["radii"])
-    assert frac_bad(o["color"], out["color"], rtol=RTOL, atol_scale=1e-6) == 0.0
+    ref = Reference(f"channel_counts[{C}-{W}-{H}]")
+    if ref.recording:
+        out = _ref_forward(_ref("chn"), sd, cm, C, True, bg)
+        ref.put("radii", out["radii"])
+        ref.put("color", out["color"])
+        del out
+    assert ref.equal("radii", o["radii"])
+    assert ref.frac_bad("color", o["color"], rtol=RTOL, atol_scale=1e-6) == 0.0
     dL = torch.as_tensor(np.random.default_rng(C).standard_normal((C, H, W)).astype(np.float32), device=dev)
     (o["color"] * dL).sum().backward()
     g = sc["features"].grad

@@ -5,9 +5,10 @@ import re
 
 import pytest
 import torch
+from reference_data import Reference
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF = "/root/reference"
+REF = os.environ.get("SGB_REFERENCE_TREE", "")     # the original project's source tree: read by recording runs only
 CHN_FIELDS = ("image_height", "image_width", "tanfovx", "tanfovy", "bg", "scale_modifier", "viewmatrix",
               "projmatrix", "sh_degree", "campos", "prefiltered", "debug", "num_channels")
 
@@ -25,11 +26,14 @@ def test_settings_fields_match_reference():
     from semantic_gaussians_b200 import rgbd_rasterization as rgbd
     assert chn.GaussianRasterizationSettings._fields == CHN_FIELDS
     assert rgbd.GaussianRasterizationSettings._fields == CHN_FIELDS[:-1]
-    if os.path.isdir(REF):
-        assert chn.GaussianRasterizationSettings._fields == _ref_settings_fields(
-            f"{REF}/submodules/channel-rasterization/channel_rasterization/__init__.py")
-        assert rgbd.GaussianRasterizationSettings._fields == _ref_settings_fields(
-            f"{REF}/submodules/rgbd-rasterization/rgbd_rasterization/__init__.py")
+    ref = Reference("python_api")
+    if ref.recording:
+        ref.put("channel_settings_fields", _ref_settings_fields(
+            f"{REF}/submodules/channel-rasterization/channel_rasterization/__init__.py"))
+        ref.put("rgbd_settings_fields", _ref_settings_fields(
+            f"{REF}/submodules/rgbd-rasterization/rgbd_rasterization/__init__.py"))
+    assert ref.equal("channel_settings_fields", chn.GaussianRasterizationSettings._fields)
+    assert ref.equal("rgbd_settings_fields", rgbd.GaussianRasterizationSettings._fields)
 
 
 def test_module_surface():
@@ -73,13 +77,17 @@ def test_eval_sh_matches_reference_python():
     torch.manual_seed(0)
     sh = torch.randn(50, 3, 16)
     d = torch.nn.functional.normalize(torch.randn(50, 3), dim=1)
-    if os.path.isdir(REF):
+    ref = Reference("eval_sh")
+    if ref.recording:
         import importlib.util
         spec = importlib.util.spec_from_file_location("ref_sh_utils", f"{REF}/utils/sh_utils.py")
         mod = importlib.util.module_from_spec(spec)
         spec.loader.exec_module(mod)
         for deg in range(4):
-            assert torch.allclose(eval_sh(deg, sh, d), mod.eval_sh(deg, sh, d), rtol=1e-6, atol=1e-6)
+            ref.put(f"degree_{deg}", mod.eval_sh(deg, sh, d))
+    for deg in range(4):
+        ours, want, _ = ref.pair(f"degree_{deg}", eval_sh(deg, sh, d))    # all 150 values are stored
+        assert torch.allclose(ours, want, rtol=1e-6, atol=1e-6)
     assert eval_sh(0, sh, d).shape == (50, 3)
 
 
